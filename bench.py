@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DEVA propagation hot path on B200 (contract: see the task statement / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], "c3"): synthetic 1080p frames (padded 1088x1920, Q = 8160 query
 positions), 16 objects, memory bank pre-filled to 10 000 slots, full encode -> read -> decode per frame
@@ -22,6 +22,8 @@ Printed JSON line: metric/value/unit/... plus
   clocks        SM clock / throttle reasons sampled with nvidia-smi during the timed region.
 ``--impl reference`` times the reference's own ``DEVAInferenceCore.step`` on the host cores (``oracle/_ref``; the
 oracle port only when the staged copy is missing).
+``--dump-outputs DIR`` writes what the last timed step returned (see dump_outputs) so that two builds can be compared
+output for output: every input is seeded, so the same arguments give the same inputs.
 """
 import argparse
 import json
@@ -31,6 +33,7 @@ import sys
 import tempfile
 import time
 
+sys.dont_write_bytecode = True  # the tree may be read-only; the bench writes nothing into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, 'tracking-anything-with-deva_b200')
 for _p in (ROOT, PKG):
@@ -86,6 +89,28 @@ def synth_mask(wl):
         y0, x0 = int((r + 0.15) * h / rows), int((c + 0.15) * w / cols)
         m[y0:y0 + int(0.6 * h / rows), x0:x0 + int(0.6 * w / cols)] = i + 1
     return m
+
+
+DUMP_LIMIT = 60 << 20  # bytes of array data in all files of --dump-outputs: the dump stays under 64 MB
+
+
+def dump_outputs(path, outputs, limit=DUMP_LIMIT, seed=0):
+    """Write ``outputs`` (name -> probabilities [C, H, W]) as float32 ``path/<name>.npy``.  When they exceed ``limit``
+    bytes together, each is stored as [C, S] instead: the same S pixel positions of every output, drawn with a fixed seed
+    and kept in raster order, S as large as the limit allows."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    per_pixel = sum(4 * t.shape[0] for t in outputs.values())
+    sample = {}
+    for name, t in outputs.items():
+        x = t.detach().float()
+        hw = x[0].numel()
+        if per_pixel * max(u[0].numel() for u in outputs.values()) > limit:
+            if hw not in sample:
+                g = torch.Generator().manual_seed(seed)
+                sample[hw] = torch.randperm(hw, generator=g)[:limit // per_pixel].sort().values
+            x = x.reshape(x.shape[0], hw)[:, sample[hw].to(x.device)]
+        np.save(os.path.join(path, name + '.npy'), x.cpu().numpy())
 
 
 def read_flops(wl, q):
@@ -249,8 +274,7 @@ class ClipSet:
         self.frames_host = self.clips[0].frames_host
 
     def step_resident(self):
-        for c in self.clips:
-            c.step_resident()
+        return [c.step_resident() for c in self.clips]
 
     def step_e2e(self):
         for c in self.clips:
@@ -275,11 +299,13 @@ def timed(fn, steps, dist_on):
     gc.disable()  # no collector pause between two launches of the timed region
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     del HOST_MS[:]
+    out = None
     t0 = time.perf_counter()
     e0.record()
     for _ in range(steps):
         h0 = time.perf_counter()
-        fn()
+        out = None  # keep the last step's result without extending the life of an earlier one into the next step
+        out = fn()
         HOST_MS.append((time.perf_counter() - h0) * 1e3)
     e1.record()
     torch.cuda.synchronize()
@@ -291,7 +317,7 @@ def timed(fn, steps, dist_on):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dist.barrier()
         ms, wall = float(t[0]), float(t[1])
-    return ms, wall
+    return ms, wall, out
 
 
 def pin_to_gpu_numa_node(gpu_index):
@@ -349,22 +375,26 @@ def run_ours(args):
         sampler.mark()
     clip.core.memory.read_events = []
     l0 = nat.launch_count()
-    ms, wall = timed(clip.step_resident, args.steps, dist_on)
+    ms, wall, last = timed(clip.step_resident, args.steps, dist_on)
     launches = nat.launch_count() - l0
     ev = clip.core.memory.read_events
     clip.core.memory.read_events = None
     read_ms = sum(a.elapsed_time(b) for a, b in ev) / max(len(ev), 1)
     clocks = sampler.stop() if sampler else None
     host_ms = sorted(HOST_MS)
+    if args.dump_outputs and rank == 0:  # this rank's clips
+        dump_outputs(args.dump_outputs, {f'prob_clip{i:02d}': p for i, p in zip(clip.ids, last)} if 'clips' in wl
+                     else {'prob': last})
+    del last
 
     for _ in range(2):
         clip.step_e2e()
-    ms_e2e, _ = timed(clip.step_e2e, args.steps, dist_on)
+    ms_e2e, _, _ = timed(clip.step_e2e, args.steps, dist_on)
     ms_e2e_io = 0.0
     if not args.quick:
         for _ in range(2):
             clip.step_e2e_fused_io()
-        ms_e2e_io, _ = timed(clip.step_e2e_fused_io, args.steps, dist_on)
+        ms_e2e_io, _, _ = timed(clip.step_e2e_fused_io, args.steps, dist_on)
 
     # conv-stack roofline: a separate short pass with CUDA events around every conv launch (not part of `value`)
     from deva.model import native_ops
@@ -806,7 +836,7 @@ def run_reference_gpu(args):
 if __name__ == '__main__':
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=10, help='timed steps (frames) of the measured path')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference', 'reference_gpu'])
     ap.add_argument('--ref-objects', type=int, default=1,
@@ -817,7 +847,11 @@ if __name__ == '__main__':
     ap.add_argument('--no-torch-baseline', action='store_true', help='skip the stock-PyTorch-on-GPU comparison pass')
     ap.add_argument('--no-c5-leg', action='store_true',
                     help='N > 1 only: skip the bank-sharded single-video leg (workload c5 on the same ranks, key bank_sharded_c5)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step to DIR/<name>.npy '
+                    '(float32, at most 64 MB in all: a fixed, seeded sample of the pixels of a larger output)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.impl == 'reference':
         run_reference(a)
     elif a.impl == 'reference_gpu':

@@ -1,23 +1,25 @@
-"""Mint golden fixtures by running the UNMODIFIED reference on CPU (build container only).
+"""Mint golden fixtures by running the UNMODIFIED reference on CPU.
 
-    python tests/golden/make_golden.py
+    DEVA_REFERENCE_ROOT=<checkout of hkchengrex/Tracking-Anything-with-DEVA @ 404a112> python tests/golden/make_golden.py
 
-Imports hkchengrex/Tracking-Anything-with-DEVA read-only from /root/reference with the three
-shims of SURVEY.md section 8(c): a stub ``pulp`` module, ``pretrained=False`` ResNets, nothing
-else.  Writes small fixtures next to this file; they pin ``oracle/`` (tests/test_oracle_golden.py)
-and, through it, the CUDA path.  /root/reference does not exist on the GPU box, so nothing at
-test/bench time runs this script.
+Imports the reference read-only from that checkout with the three shims of SURVEY.md section 8(c):
+a stub ``pulp`` module, ``pretrained=False`` ResNets, nothing else.  Writes small fixtures next to
+this file; they pin ``oracle/`` (tests/test_oracle_golden.py) and, through it, the CUDA path.
+Nothing at test/bench time runs this script: the tests need only what it wrote.
 """
 import json
 import os
+import shutil
 import sys
 import types
+import zipfile
 
 sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.modules['pulp'] = types.ModuleType('pulp')
-sys.path.insert(0, '/root/reference')
+REF = os.environ['DEVA_REFERENCE_ROOT']
+sys.path.insert(0, REF)
 
 import numpy as np
 import torch
@@ -40,6 +42,8 @@ _spec = importlib.util.spec_from_file_location(
     'b200_param_spec', os.path.join(ROOT, 'tracking-anything-with-deva_b200', 'deva', 'model', 'param_spec.py'))
 param_spec = importlib.util.module_from_spec(_spec)
 _spec.loader.exec_module(param_spec)
+sys.path.append(ROOT)
+from oracle import fixtures  # noqa: E402  (the compact storage of the two clip fixtures)
 
 CFG = dict(key_dim=64, value_dim=512, pix_feat_dim=512, mem_every=5, enable_long_term=True,
            chunk_size=-1, top_k=30, enable_long_term_count_usage=True, max_mid_term_frames=10,
@@ -48,8 +52,11 @@ torch.set_grad_enabled(False)
 
 
 def save(name, **arrays):
-    np.savez_compressed(os.path.join(HERE, name), **{k: (v.numpy() if torch.is_tensor(v) else v)
-                                                      for k, v in arrays.items()})
+    """np.savez_compressed's layout at the strongest deflate level (keeps every fixture under 1 MB)."""
+    with zipfile.ZipFile(os.path.join(HERE, name), 'w', zipfile.ZIP_DEFLATED, compresslevel=9) as zf:
+        for k, v in arrays.items():
+            with zf.open(k + '.npy', 'w', force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asarray(v.numpy() if torch.is_tensor(v) else v), allow_pickle=False)
     print('wrote', name, {k: tuple(v.shape) for k, v in arrays.items() if hasattr(v, 'shape')})
 
 
@@ -137,10 +144,8 @@ def golden_vos():
     net.load_weights(sd)
     np.random.seed(42)
     core = DEVAInferenceCore(net, cfg)
-    g = torch.Generator().manual_seed(11)
     H, W, T = 80, 96, 16
-    base = torch.randn(3, H, W, generator=g)
-    frames = torch.stack([base + 0.2 * torch.randn(3, H, W, generator=g) for _ in range(T)])
+    frames = torch.from_numpy(fixtures.vos_frames(11, T, H, W))
     m0 = torch.zeros(H, W, dtype=torch.long); m0[6:40, 6:44] = 1; m0[44:76, 40:90] = 2
     m6 = torch.zeros(H, W, dtype=torch.long); m6[10:34, 56:92] = 7
     probs, sizes = [], []
@@ -154,9 +159,13 @@ def golden_vos():
         probs.append(p.clone())
         mem = core.memory
         sizes.append({str(b): [mem.work_mem.size(b), mem.long_mem.size(b)] for b in mem.work_mem.buckets})
-    arrays = {f'prob_{t:02d}': p for t, p in enumerate(probs)}
-    save('vos_steps.npz', frames=frames, mask0=m0, mask6=m6, **arrays)
-    json.dump({'config': cfg, 'sizes': sizes}, open(os.path.join(HERE, 'vos_steps.json'), 'w'))
+    # frames are regenerated from their seed by oracle.fixtures.vos_steps; probabilities as 16-bit fixed point
+    arrays = {f'prob_{t:02d}': (p.double() * fixtures.PROB_SCALE).round().to(torch.int32).numpy().astype(np.uint16)
+              for t, p in enumerate(probs)}
+    save('vos_steps.npz', mask0=m0.to(torch.uint8), mask6=m6.to(torch.uint8), **arrays)
+    json.dump({'config': cfg, 'sizes': sizes,
+               'frames': {'seed': 11, 'shape': [T, H, W], 'sha256': fixtures.sha256(frames.numpy())}},
+              open(os.path.join(HERE, 'vos_steps.json'), 'w'))
     print('  sizes', sizes[-1], 'prob range', float(probs[-1].min()), float(probs[-1].max()))
 
 
@@ -365,7 +374,7 @@ def golden_config1():
     fp32 values is NOT used: kept fp32 so the 1e-3 contract can be checked)."""
     from PIL import Image
     from torchvision import transforms
-    root = '/root/reference/example/vos'
+    root = os.path.join(REF, 'example', 'vos')
     vid = 'bmx-trees'
     names = sorted(os.listdir(os.path.join(root, 'JPEGImages', vid)))
     norm = transforms.Compose([transforms.ToTensor(),
@@ -381,7 +390,7 @@ def golden_config1():
     net.load_weights(param_spec.synthetic_state_dict(seed=1))
     np.random.seed(42)
     core = DEVAInferenceCore(net, cfg)
-    arrays = dict(frames_u8=frames_u8, mask0=mask0.astype(np.uint8))
+    arrays = dict(mask0=mask0.astype(np.uint8))  # the frames are stored as the example's JPEG files
     for t in range(vid_length):
         image = norm(Image.fromarray(frames_u8[t]))
         mask = torch.from_numpy(mask0.astype(np.int64)) if t == 0 else None
@@ -394,7 +403,11 @@ def golden_config1():
         print('  config1 t', t, 'prob', tuple(prob.shape), 'ids', np.unique(arrays[f'ids_{t}']).tolist(),
               'confident', float(((top2[0] - top2[1]) > 0.05).float().mean()))
     save('config1_vos.npz', **arrays)
-    json.dump({'config': cfg, 'labels': labels, 'frames': names, 'video': vid},
+    os.makedirs(os.path.join(HERE, vid), exist_ok=True)
+    for n in names:
+        shutil.copyfile(os.path.join(root, 'JPEGImages', vid, n), os.path.join(HERE, vid, n))
+    json.dump({'config': cfg, 'labels': labels, 'frames': names, 'video': vid,
+               'frames_u8_sha256': fixtures.sha256(frames_u8)},
               open(os.path.join(HERE, 'config1_vos.json'), 'w'))
 
 

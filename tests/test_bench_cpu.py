@@ -83,3 +83,25 @@ def test_workload_table_matches_baseline_json():
     assert (c3['h'], c3['w'], c3['k'], c3['n']) == (1080, 1920, 16, 10000)     # configs[2]
     assert (c5['k'], c5['n'], c5.get('sharded')) == (32, 50000, True)          # configs[4]
     assert bench.WORKLOADS['c4']['clips'] == 64                                 # configs[3]
+
+
+def test_dump_outputs_are_float32_bounded_and_repeatable(tmp_path):
+    """--dump-outputs: a small output is written whole as float32; one over the limit becomes [C, S], S pixel positions
+    in raster order, the same ones on every run."""
+    import numpy as np
+    import torch
+    import bench
+    small = torch.rand(3, 4, 5, dtype=torch.float16)
+    bench.dump_outputs(str(tmp_path / 'a'), {'prob': small})
+    got = np.load(tmp_path / 'a' / 'prob.npy')
+    assert got.dtype == np.float32 and np.array_equal(got, small.float().numpy())
+    big = torch.rand(17, 30, 40)
+    limit = 17 * 4 * 500
+    for d in ('b', 'c'):
+        bench.dump_outputs(str(tmp_path / d), {'prob': big}, limit=limit)
+    b, c = np.load(tmp_path / 'b' / 'prob.npy'), np.load(tmp_path / 'c' / 'prob.npy')
+    assert b.dtype == np.float32 and b.shape == (17, 500) and b.nbytes <= limit and np.array_equal(b, c)
+    column = {v: i for i, v in enumerate(big[0].flatten().tolist())}
+    idx = [column[v] for v in b[0].tolist()]
+    assert idx == sorted(set(idx))
+    assert np.array_equal(b, big.reshape(17, -1).numpy()[:, idx])

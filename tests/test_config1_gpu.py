@@ -5,27 +5,20 @@ unmodified reference recorded by tests/golden/make_golden.py::golden_config1.  T
 the suite (everything else is <= 100x150 synthetic frames)."""
 import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
+from oracle import fixtures
+
 pytestmark = pytest.mark.gpu
 
 
 def _reference_cross_device_deviation(golden_dir):
-    """max |prob(reference on this GPU, fp32, no TF32) - prob(reference on the CPU, the fixture)| on the lattice, or None
-    when the staged reference (oracle/_ref) is not present.  See tests/golden/ref_on_gpu.py."""
-    root = os.path.dirname(os.path.dirname(golden_dir))
-    if not os.path.isfile(os.path.join(root, 'oracle', '_ref', 'deva', 'inference', 'inference_core.py')):
-        return None
-    r = subprocess.run([sys.executable, os.path.join(golden_dir, 'ref_on_gpu.py')], capture_output=True, text=True, timeout=600)
-    for line in reversed(r.stdout.strip().splitlines()):
-        if line.startswith('{'):
-            return json.loads(line)['worst']
-    raise RuntimeError('ref_on_gpu.py failed: ' + r.stderr[-400:])
+    """max |prob(reference on a B200, fp32, no TF32) - prob(reference on the CPU, the fixture)| on the lattice, as
+    measured by tests/golden/ref_on_gpu.py and stored next to the fixture, with the device it was measured on."""
+    return json.load(open(os.path.join(golden_dir, 'config1_ref_on_gpu.json')))
 
 
 @pytest.mark.parametrize('backend,tol', [('native', 1e-3), ('torch', 1e-3)])
@@ -35,8 +28,7 @@ def test_example_vos_clip_matches_reference(golden_dir, synthetic_sd, backend, t
     from deva.model.network import DEVA
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
-    g = np.load(os.path.join(golden_dir, 'config1_vos.npz'))
-    meta = json.load(open(os.path.join(golden_dir, 'config1_vos.json')))
+    g, meta = fixtures.config1_vos(golden_dir)
     net = DEVA(meta['config'])
     net.conv_backend = backend
     net = net.cuda().eval()
@@ -73,8 +65,8 @@ def test_example_vos_clip_matches_reference(golden_dir, synthetic_sd, backend, t
         assert float(decided.float().mean()) > 0.5 or t > 0
     floor = _reference_cross_device_deviation(golden_dir)
     print(f'[{backend}] example/vos clip: max |prob - reference| on the lattice = {worst:.3e}, fraction of lattice points '
-          f'over {tol:g}: {over:.2e}; unmodified reference on this GPU vs its own CPU run: '
-          f'{floor if floor is None else format(floor, ".3e")}')
+          f'over {tol:g}: {over:.2e}; unmodified reference on {floor["device"]} ({floor["power_limit_w"]} W limit) vs '
+          f'its own CPU run: {floor["worst"]:.3e}')
     # Real-image keys put the top-30 cut of the memory read (memory_utils.py:56-64) through nearly tied similarities:
     # on this clip 12 % of the queries have their 30th and 31st similarity within 1e-4, some within the ~4e-6 rounding
     # noise of the fp32 similarity itself, and the 30th member still carries 1/30 of the softmax weight.  Which member

@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import fixtures
 from oracle import memory_math as mm
 from oracle import network as net
 from oracle.core import CoreOracle
@@ -62,8 +63,8 @@ def test_network_stages_match_reference(golden_dir, synthetic_sd):
 
 
 def test_vos_steps_match_reference(golden_dir, synthetic_sd):
-    g = _load(golden_dir, 'vos_steps.npz')
-    meta = json.load(open(os.path.join(golden_dir, 'vos_steps.json')))
+    arrays, meta = fixtures.vos_steps(golden_dir)
+    g = {k: torch.from_numpy(v) for k, v in arrays.items()}
     np.random.seed(42)
     core = CoreOracle(synthetic_sd, meta['config'])
     T = g['frames'].shape[0]

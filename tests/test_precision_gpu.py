@@ -95,15 +95,13 @@ def test_conv_weight_lo_mode_with_rank1_and_residual():
 
 def test_fast_plan_is_still_available(golden_dir, synthetic_sd, monkeypatch):
     """DEVA_B200_PRECISION=fast: single fp16 operands everywhere (the round-1 stack) stays within 2.5e-3."""
-    import json
-    import os
-
     import numpy as np
     from deva.inference.inference_core import DEVAInferenceCore
     from deva.model.network import DEVA
+    from oracle import fixtures
     monkeypatch.setenv('DEVA_B200_PRECISION', 'fast')
-    g = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(golden_dir, 'vos_steps.npz')).items()}
-    meta = json.load(open(os.path.join(golden_dir, 'vos_steps.json')))
+    arrays, meta = fixtures.vos_steps(golden_dir)
+    g = {k: torch.from_numpy(v) for k, v in arrays.items()}
     np.random.seed(42)
     net = DEVA(meta['config'])
     net.conv_backend = 'native'

@@ -1,10 +1,9 @@
 """GPU parity of the full DEVAInferenceCore.step path against reference-minted golden frames."""
-import json
-import os
-
 import numpy as np
 import pytest
 import torch
+
+from oracle import fixtures
 
 pytestmark = pytest.mark.gpu
 
@@ -26,8 +25,8 @@ def _core(cfg, sd, backend):
 def test_vos_clip_matches_reference(golden_dir, synthetic_sd, backend, tol):
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
-    g = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(golden_dir, 'vos_steps.npz')).items()}
-    meta = json.load(open(os.path.join(golden_dir, 'vos_steps.json')))
+    arrays, meta = fixtures.vos_steps(golden_dir)
+    g = {k: torch.from_numpy(v) for k, v in arrays.items()}
     np.random.seed(42)
     core = _core(meta['config'], synthetic_sd, backend)
     T = g['frames'].shape[0]

@@ -1,7 +1,6 @@
 """GPU diagnostic: where does the product differ from the CPU oracle on the real-image clip (config 1)?  Steps the
 product core (both conv backends) and oracle.core.CoreOracle side by side and compares, frame by frame: key / shrinkage /
 selection, the memory read-out, the aggregated logits and the probabilities (each pipeline on its own state)."""
-import json
 import os
 import sys
 
@@ -14,6 +13,7 @@ sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
 from deva.inference.inference_core import DEVAInferenceCore  # noqa: E402
 from deva.model.network import DEVA  # noqa: E402
 from deva.model.param_spec import synthetic_state_dict  # noqa: E402
+from oracle import fixtures  # noqa: E402
 from oracle import network as onet  # noqa: E402
 from oracle.core import CoreOracle  # noqa: E402
 
@@ -28,8 +28,7 @@ def rel(a, b):
 
 
 def main():
-    g = np.load(os.path.join(ROOT, 'tests/golden/config1_vos.npz'))
-    meta = json.load(open(os.path.join(ROOT, 'tests/golden/config1_vos.json')))
+    g, meta = fixtures.config1_vos()
     mean = torch.tensor([0.485, 0.456, 0.406]).view(3, 1, 1)
     std = torch.tensor([0.229, 0.224, 0.225]).view(3, 1, 1)
     frames = [((torch.from_numpy(g['frames_u8'][t]).permute(2, 0, 1).float() / 255) - mean) / std for t in range(4)]

@@ -1,7 +1,6 @@
 """GPU experiment: max / rms |prob - reference| over the golden clip under different per-layer precision plans
 (DEVA_B200_PLAN overrides on top of the default 'parity' plan).  Calibrates tools/precision_plan.py's CPU emulation
 against the kernels.   python tools/plan_sweep.py [plan ...]   (a plan is a DEVA_B200_PLAN string; '' = default)"""
-import json
 import os
 import sys
 
@@ -9,14 +8,16 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
 from deva.inference.inference_core import DEVAInferenceCore  # noqa: E402
 from deva.model.network import DEVA  # noqa: E402
 from deva.model.param_spec import synthetic_state_dict  # noqa: E402
+from oracle import fixtures  # noqa: E402
 
 torch.set_grad_enabled(False)
-G = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(ROOT, 'tests/golden/vos_steps.npz')).items()}
-META = json.load(open(os.path.join(ROOT, 'tests/golden/vos_steps.json')))
+_ARRAYS, META = fixtures.vos_steps()
+G = {k: torch.from_numpy(v) for k, v in _ARRAYS.items()}
 SD = {k: v.cuda() for k, v in synthetic_state_dict(seed=1).items()}
 
 DEFAULT_PLANS = [

@@ -6,7 +6,6 @@ pass (hi/lo weights) or a hi/lo activation operand buys the most.
   python tools/precision_layers.py scan            # one run per (layer, w|x)
   python tools/precision_layers.py plan a,b,c ...  # evaluate a named configuration
 """
-import json
 import os
 import sys
 
@@ -17,6 +16,7 @@ import torch.nn.functional as F
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
+from oracle import fixtures  # noqa: E402
 from oracle import memory_math as mm  # noqa: E402
 from oracle import network as net  # noqa: E402
 from oracle.core import CoreOracle  # noqa: E402
@@ -82,8 +82,8 @@ net._gru = gru
 net.encode_mask = encode_mask
 mm.readout = readout
 
-G = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(ROOT, 'tests/golden/vos_steps.npz')).items()}
-META = json.load(open(os.path.join(ROOT, 'tests/golden/vos_steps.json')))
+_ARRAYS, META = fixtures.vos_steps()
+G = {k: torch.from_numpy(v) for k, v in _ARRAYS.items()}
 SD = synthetic_state_dict(seed=1)
 REF = None
 

@@ -7,7 +7,6 @@ which tensors travel as hi/lo pairs and which convs consume the lo part of their
 
     python tools/precision_plan.py            # the plans listed in PLANS below
 """
-import json
 import os
 import sys
 
@@ -18,6 +17,7 @@ import torch.nn.functional as F
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
+from oracle import fixtures  # noqa: E402
 from oracle import memory_math as mm  # noqa: E402
 from oracle import network as net  # noqa: E402
 from oracle.core import CoreOracle  # noqa: E402
@@ -177,8 +177,8 @@ net.segment = segment
 net.encode_mask = encode_mask
 mm.readout = readout
 
-G = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(ROOT, 'tests/golden/vos_steps.npz')).items()}
-META = json.load(open(os.path.join(ROOT, 'tests/golden/vos_steps.json')))
+_ARRAYS, META = fixtures.vos_steps()
+G = {k: torch.from_numpy(v) for k, v in _ARRAYS.items()}
 SD = synthetic_state_dict(seed=1)
 REF = None
 

@@ -1,10 +1,11 @@
 """CPU study: where does fp16 storage hurt?  Monkeypatches the oracle network so that selected
 activations / weights are rounded to fp16 like the native engine does, and replays the golden clip."""
-import json, os, sys
+import os, sys
 import numpy as np, torch
 import torch.nn.functional as F
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
+from oracle import fixtures
 from oracle import network as net
 from oracle import memory_math as mm
 from oracle.core import CoreOracle
@@ -58,8 +59,8 @@ net.encode_mask = encode_mask
 mm.readout = readout
 
 def run(tag):
-    g = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(ROOT, 'tests/golden/vos_steps.npz')).items()}
-    meta = json.load(open(os.path.join(ROOT, 'tests/golden/vos_steps.json')))
+    arrays, meta = fixtures.vos_steps()
+    g = {k: torch.from_numpy(v) for k, v in arrays.items()}
     np.random.seed(42)
     core = CoreOracle(synthetic_state_dict(seed=1), meta['config'])
     worst = 0

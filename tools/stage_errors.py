@@ -8,11 +8,13 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
 from deva.model.engine import Engine  # noqa: E402
 from deva.model.native_engine import NativeEngine  # noqa: E402
 from deva.model.param_spec import synthetic_state_dict  # noqa: E402
 from deva.utils.tensor_utils import pad_divide_by  # noqa: E402
+from oracle import fixtures  # noqa: E402
 
 torch.backends.cudnn.allow_tf32 = False
 torch.backends.cuda.matmul.allow_tf32 = False
@@ -30,7 +32,7 @@ def report(name, a, b):
 
 def main():
     dev = 'cuda'
-    g = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(ROOT, 'tests/golden/vos_steps.npz')).items()}
+    g = {k: torch.from_numpy(v) for k, v in fixtures.vos_steps()[0].items()}
     sd = {k: v.to(dev) for k, v in synthetic_state_dict(seed=1).items()}
     ref, nat = Engine(sd), NativeEngine(sd)
     image, _ = pad_divide_by(g['frames'][0].to(dev), 16)

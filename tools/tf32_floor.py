@@ -10,10 +10,12 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tracking-anything-with-deva_b200'))
 from deva.inference.inference_core import DEVAInferenceCore  # noqa: E402
 from deva.model.network import DEVA  # noqa: E402
 from deva.model.param_spec import synthetic_state_dict  # noqa: E402
+from oracle import fixtures  # noqa: E402
 
 torch.set_grad_enabled(False)
 
@@ -21,9 +23,8 @@ torch.set_grad_enabled(False)
 def run(backend, tf32):
     torch.backends.cudnn.allow_tf32 = tf32
     torch.backends.cuda.matmul.allow_tf32 = False
-    gd = os.path.join(ROOT, 'tests', 'golden')
-    g = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(gd, 'vos_steps.npz')).items()}
-    meta = json.load(open(os.path.join(gd, 'vos_steps.json')))
+    arrays, meta = fixtures.vos_steps()
+    g = {k: torch.from_numpy(v) for k, v in arrays.items()}
     np.random.seed(42)
     net = DEVA(meta['config'])
     net.conv_backend = backend

@@ -1,5 +1,5 @@
 """GPU probe: how often, and by how much, does the fused similarity/top-k kernel pick a different top-30 than exact
-arithmetic on REAL-image keys (example clip of tests/golden/config1_vos.npz)?  Memory = keys of frame 0, queries = keys
+arithmetic on REAL-image keys (example clip of tests/golden/config1_vos.*)?  Memory = keys of frame 0, queries = keys
 of frame 1, both from the cuDNN fp32 engine; ground truth = fp64 similarity on the CPU.  For every query whose set
 differs it reports delta = sim64(best excluded) - sim64(worst included): the similarity error that caused the swap."""
 import os
@@ -15,6 +15,7 @@ from deva import _native as nat  # noqa: E402
 from deva.model.engine import Engine  # noqa: E402
 from deva.model.param_spec import synthetic_state_dict  # noqa: E402
 from deva.utils.tensor_utils import pad_divide_by  # noqa: E402
+from oracle import fixtures  # noqa: E402
 from oracle import memory_math as mm  # noqa: E402
 
 torch.set_grad_enabled(False)
@@ -23,7 +24,7 @@ torch.backends.cuda.matmul.allow_tf32 = False
 
 
 def main():
-    g = np.load(os.path.join(ROOT, 'tests/golden/config1_vos.npz'))
+    g, _ = fixtures.config1_vos()
     mean = torch.tensor([0.485, 0.456, 0.406]).view(3, 1, 1)
     std = torch.tensor([0.229, 0.224, 0.225]).view(3, 1, 1)
     eng = Engine({k: v.cuda() for k, v in synthetic_state_dict(seed=1).items()})
