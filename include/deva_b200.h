@@ -27,9 +27,11 @@
 extern "C" {
 #endif
 
-/* v11: deva_b200_cbam / deva_b200_cbam_split take a larger scratch buffer (64 pooling slices) and require c = 8 x a divisor
+/* v12: deva_b200_resize_rgb8, deva_b200_resize_rgb8_workspace_bytes, deva_b200_resize_aa_weights and
+ * deva_b200_resize_labels (frames and first-frame masks resized to the evaluation size on the device).
+ * v11: deva_b200_cbam / deva_b200_cbam_split take a larger scratch buffer (64 pooling slices) and require c = 8 x a divisor
  * of 256; deva_b200_conv2d requires cout_pad <= 2048 (<= 1024 with a rank-1 input): the layer's bias lives in shared memory. */
-#define DEVA_B200_ABI_VERSION 11
+#define DEVA_B200_ABI_VERSION 12
 #define DEVA_B200_LIST_PITCH 32 /* row pitch of top-k outputs == max supported top_k */
 #define DEVA_B200_MAX_GROUPS 256 /* objects per deva_b200_readout call */
 
@@ -287,6 +289,31 @@ DEVA_B200_API int deva_b200_ingest_rgb8(const uint8_t* src, float* dst, int h, i
  * out_i64 [out_h, out_w] (either may be NULL). */
 DEVA_B200_API int deva_b200_prob_to_ids(const float* prob, int c, int h, int w, int out_h, int out_w, int flip,
                                         const int32_t* lut, uint8_t* out_u8, int64_t* out_i64, deva_stream_t stream);
+
+/* Frame u8 [h, w, 3] (RGB interleaved) -> fp32 [3, out_h, out_w]: ToTensor + Normalize per source pixel as in
+ * deva_b200_ingest_rgb8, then a resize to the evaluation size.
+ *  - DEVA_B200_RESIZE_READER: torchvision Resize(bilinear, antialias=True) after the normalisation
+ *    (deva/inference/data/video_reader.py:141-145): separable triangle filter, rows first into the fp32 workspace
+ *    `ws` [3, h, out_w], then columns; the tap weights are bit-identical to torch's float32 CPU ones.
+ *  - DEVA_B200_RESIZE_DEMO: F.interpolate(bilinear, align_corners=False) (deva/inference/demo_utils.py:10-19);
+ *    `ws` is unused and may be NULL.
+ * The caller picks out_h / out_w (torchvision's Resize(size) rule for the reader, int(h * size / min(h, w)) for the
+ * demo) and, for the reader, skips the call when they equal h / w: torchvision returns such an image unresized. */
+#define DEVA_B200_RESIZE_READER 0
+#define DEVA_B200_RESIZE_DEMO 1
+DEVA_B200_API size_t deva_b200_resize_rgb8_workspace_bytes(int h, int w, int out_h, int out_w, int mode);
+DEVA_B200_API int deva_b200_resize_rgb8(const uint8_t* src, float* dst, float* ws, int h, int w, int out_h, int out_w,
+                                        int mode, const float mean[3], const float std[3], deva_stream_t stream);
+/* HOST: the antialiased tap tables deva_b200_resize_rgb8 computes on the fly for one axis n_in -> n_out: output i
+ * reads x0[i] .. x0[i] + n[i] - 1 with weights w[i * max_taps + j] (zero past n[i]).  Fails when max_taps is below
+ * 2 * ceil(max(n_in / n_out, 1)) + 1.  Needs no GPU. */
+DEVA_B200_API int deva_b200_resize_aa_weights(int n_in, int n_out, int max_taps, int32_t* x0, int32_t* n, float* w);
+/* Palette mask u8 [h, w] -> int64 [out_h, out_w], dst[y, x] = src[src_y[y], src_x[x]] (0 where either index is
+ * negative).  With Pillow's NEAREST tables (INTEGRATION.md) this is transforms.Resize(size, NEAREST) on the 'P' image
+ * followed by torch.LongTensor (video_reader.py:147-150, 211-214), bit for bit.  src_y int32 [out_h], src_x int32
+ * [out_w]. */
+DEVA_B200_API int deva_b200_resize_labels(const uint8_t* src, int64_t* dst, int h, int w, int out_h, int out_w,
+                                          const int32_t* src_y, const int32_t* src_x, deva_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -248,5 +248,21 @@ DEVA_B200_API int deva_b200_prob_to_ids(const float* prob, int c, int h, int w, 
                                         const int32_t* lut, uint8_t* out_u8, int64_t* out_i64, deva_stream_t stream) {
   return ew_prob_to_ids(prob, c, h, w, out_h, out_w, flip, lut, out_u8, reinterpret_cast<long long*>(out_i64), S(stream));
 }
+static_assert(RESIZE_READER == DEVA_B200_RESIZE_READER && RESIZE_DEMO == DEVA_B200_RESIZE_DEMO, "resize modes");
+DEVA_B200_API size_t deva_b200_resize_rgb8_workspace_bytes(int h, int w, int out_h, int out_w, int mode) {
+  (void)w; (void)out_h;
+  return ew_resize_rgb8_workspace_bytes(h, out_w, mode);
+}
+DEVA_B200_API int deva_b200_resize_rgb8(const uint8_t* src, float* dst, float* ws, int h, int w, int out_h, int out_w,
+                                        int mode, const float mean[3], const float std[3], deva_stream_t stream) {
+  return ew_resize_rgb8(src, dst, ws, h, w, out_h, out_w, mode, mean, std, S(stream));
+}
+DEVA_B200_API int deva_b200_resize_aa_weights(int n_in, int n_out, int max_taps, int32_t* x0, int32_t* n, float* w) {
+  return ew_resize_aa_weights(n_in, n_out, max_taps, x0, n, w);
+}
+DEVA_B200_API int deva_b200_resize_labels(const uint8_t* src, int64_t* dst, int h, int w, int out_h, int out_w,
+                                          const int32_t* src_y, const int32_t* src_x, deva_stream_t stream) {
+  return ew_resize_labels(src, reinterpret_cast<long long*>(dst), h, w, out_h, out_w, src_y, src_x, S(stream));
+}
 
 }  // extern "C"

@@ -941,6 +941,17 @@ ingest_rgb8_kernel(const unsigned char* __restrict__ src, float* __restrict__ ds
   dst[2 * hw + i] = __fdiv_rn(__fdiv_rn((float)p[2], 255.f) - m2, s2);
 }
 
+// Source index, neighbour step (0 at the last row / column) and the two weights of output o along one axis of an
+// align_corners=False bilinear resize with r = in / out: PyTorch's area_pixel_compute_source_index and
+// upsample_bilinear2d_out_frame arithmetic.
+__device__ __forceinline__ void bilinear_src(float r, int o, int n, int& i0, int& ip, float& l0, float& l1) {
+  const float s = fmaxf(r * (o + 0.5f) - 0.5f, 0.f);
+  i0 = (int)s;
+  ip = i0 < n - 1 ? 1 : 0;
+  l1 = s - i0;
+  l0 = 1.f - l1;
+}
+
 // prob [c, h, w] -> ids [out_h, out_w]: bilinear (align_corners = False, PyTorch's upsample_bilinear2d arithmetic),
 // flip, argmax (first maximum), id remap.  One thread per output pixel, channels streamed.
 __global__ void __launch_bounds__(256)
@@ -962,10 +973,10 @@ prob_to_ids_kernel(const float* __restrict__ prob, int c, int h, int w, int out_
       if (v > best_v) { best_v = v; best = k; }
     }
   } else {
-    const float sy = fmaxf(rh * (oy + 0.5f) - 0.5f, 0.f), sx = fmaxf(rw * (ox + 0.5f) - 0.5f, 0.f);
-    const int y0 = (int)sy, x0 = (int)sx;
-    const int yp = y0 < h - 1 ? 1 : 0, xp = x0 < w - 1 ? 1 : 0;
-    const float ly1 = sy - y0, ly0 = 1.f - ly1, lx1 = sx - x0, lx0 = 1.f - lx1;
+    int y0, yp, x0, xp;
+    float ly0, ly1, lx0, lx1;
+    bilinear_src(rh, oy, h, y0, yp, ly0, ly1);
+    bilinear_src(rw, ox, w, x0, xp, lx0, lx1);
     const float* p = prob + (long long)y0 * w + x0;
     best_v = -INFINITY;
     for (int k = 0; k < c; ++k) {
@@ -977,6 +988,142 @@ prob_to_ids_kernel(const float* __restrict__ prob, int c, int h, int w, int out_
   const int id = lut ? lut[best] : best;
   if (out_u8) out_u8[i] = (unsigned char)id;
   if (out_i64) out_i64[i] = id;
+}
+
+__device__ __forceinline__ float normalise_u8(unsigned char v, float m, float sd) {
+  return __fdiv_rn(__fdiv_rn((float)v, 255.f) - m, sd);
+}
+
+// u8 [h, w, 3] -> fp32 [3, out_h, out_w]: ToTensor + Normalize per source pixel, then F.interpolate(bilinear,
+// align_corners=False, antialias=False) - the demos' get_input_frame_for_deva.  One thread per output pixel.
+__global__ void __launch_bounds__(256)
+resize_bilinear_rgb8_kernel(const unsigned char* __restrict__ src, float* __restrict__ dst, int h, int w, int out_h,
+                            int out_w, float rh, float rw, float m0, float m1, float m2, float s0, float s1, float s2) {
+  const long long i = blockIdx.x * 256ll + threadIdx.x, n = (long long)out_h * out_w;
+  if (i >= n) return;
+  const int oy = (int)(i / out_w), ox = (int)(i - (long long)oy * out_w);
+  int y0, yp, x0, xp;
+  float ly0, ly1, lx0, lx1;
+  bilinear_src(rh, oy, h, y0, yp, ly0, ly1);
+  bilinear_src(rw, ox, w, x0, xp, lx0, lx1);
+  const unsigned char* p00 = src + ((long long)y0 * w + x0) * 3;
+  const unsigned char *p01 = p00 + 3 * xp, *p10 = p00 + 3ll * yp * w, *p11 = p10 + 3 * xp;
+  const float m[3] = {m0, m1, m2}, sd[3] = {s0, s1, s2};
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const float v00 = normalise_u8(p00[c], m[c], sd[c]), v01 = normalise_u8(p01[c], m[c], sd[c]);
+    const float v10 = normalise_u8(p10[c], m[c], sd[c]), v11 = normalise_u8(p11[c], m[c], sd[c]);
+    dst[c * n + i] = ly0 * (lx0 * v00 + lx1 * v01) + ly1 * (lx0 * v10 + lx1 * v11);
+  }
+}
+
+// Antialiased bilinear along one axis (in -> out), torch's _compute_weights_aa (aten/src/ATen/native/cpu/
+// UpSampleKernel.cpp) for a float32 tensor, in its own mix of fp32 values and fp64 sums: the weights come out
+// bit-identical to torch's.  Rounding scale and center to fp32 moves the taps by up to an fp32 ulp of the source
+// coordinate, which is why torch's fp32 resize differs from an fp64 one by ~1e-4 on [-2.1, 2.7] data; mirroring the
+// arithmetic keeps this kernel on torch's side of that gap.  Host and device share it (deva_b200_resize_aa_weights).
+struct AaAxis {
+  float scale, support, invscale;
+  int n_in, max_taps;
+};
+__host__ __device__ inline AaAxis aa_axis(int n_in, int n_out) {
+  AaAxis a;
+  a.n_in = n_in;
+  a.scale = (float)n_in / (float)n_out;
+  const bool down = a.scale >= 1.f;
+  a.support = down ? a.scale : 1.f;  // half the bilinear kernel width (1), stretched by scale when downscaling
+  a.invscale = down ? (float)(1.0 / (double)a.scale) : 1.f;
+  a.max_taps = (int)ceilf(a.support) * 2 + 1;
+  return a;
+}
+// window [x0, x0 + n) of output i and its fp32 center
+__host__ __device__ inline void aa_window(const AaAxis& a, int i, float& center, int& x0, int& n) {
+  center = (float)((double)a.scale * (i + 0.5));
+  const int lo = (int)((double)(center - a.support) + 0.5), hi = (int)((double)(center + a.support) + 0.5);
+  x0 = lo > 0 ? lo : 0;
+  n = (hi < a.n_in ? hi : a.n_in) - x0;
+  n = n < 0 ? 0 : (n > a.max_taps ? a.max_taps : n);
+}
+// unnormalised triangle weight of source index x
+__host__ __device__ inline float aa_tap(const AaAxis& a, float center, int x) {
+  const float t = fabsf((float)(((double)((float)x - center) + 0.5) * (double)a.invscale));
+  return t < 1.f ? 1.f - t : 0.f;
+}
+__host__ __device__ inline float aa_total(const AaAxis& a, float center, int x0, int n) {
+  float total = 0.f;
+  for (int j = 0; j < n; ++j) total += aa_tap(a, center, x0 + j);
+  return total;
+}
+// torch leaves an all-zero window unnormalised
+__host__ __device__ inline float aa_weight(const AaAxis& a, float center, int x, float total) {
+  const float t = aa_tap(a, center, x);
+  return total != 0.f ? t / total : t;
+}
+
+// Horizontal pass of the antialiased resize: u8 [h, w, 3] -> fp32 mid [3, h, out_w], each source pixel normalised
+// (ToTensor + Normalize) before it is weighted, accumulated like torch: t = v0 * w0, then t = fma(vj, wj, t).
+__global__ void __launch_bounds__(256)
+resize_aa_rows_rgb8_kernel(const unsigned char* __restrict__ src, float* __restrict__ mid, int h, int w, int out_w,
+                           AaAxis ax, float m0, float m1, float m2, float s0, float s1, float s2) {
+  const long long i = blockIdx.x * 256ll + threadIdx.x, n_mid = (long long)h * out_w;
+  if (i >= n_mid) return;
+  const int y = (int)(i / out_w), ox = (int)(i - (long long)y * out_w);
+  float center;
+  int x0, n;
+  aa_window(ax, ox, center, x0, n);
+  const float total = aa_total(ax, center, x0, n);
+  const unsigned char* p = src + ((long long)y * w + x0) * 3;
+  float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+  for (int j = 0; j < n; ++j, p += 3) {
+    const float wt = aa_weight(ax, center, x0 + j, total);
+    const float v0 = normalise_u8(p[0], m0, s0), v1 = normalise_u8(p[1], m1, s1), v2 = normalise_u8(p[2], m2, s2);
+    if (j == 0) {
+      a0 = __fmul_rn(v0, wt); a1 = __fmul_rn(v1, wt); a2 = __fmul_rn(v2, wt);
+    } else {
+      a0 = __fmaf_rn(v0, wt, a0); a1 = __fmaf_rn(v1, wt, a1); a2 = __fmaf_rn(v2, wt, a2);
+    }
+  }
+  mid[i] = a0;
+  mid[n_mid + i] = a1;
+  mid[2 * n_mid + i] = a2;
+}
+
+// Vertical pass: mid fp32 [3, h, out_w] -> dst [3, out_h, out_w], same accumulation.
+__global__ void __launch_bounds__(256)
+resize_aa_cols_kernel(const float* __restrict__ mid, float* __restrict__ dst, int h, int out_h, int out_w, AaAxis ay) {
+  const long long i = blockIdx.x * 256ll + threadIdx.x, n = (long long)out_h * out_w;
+  if (i >= n) return;
+  const int oy = (int)(i / out_w), ox = (int)(i - (long long)oy * out_w);
+  float center;
+  int y0, m;
+  aa_window(ay, oy, center, y0, m);
+  const float total = aa_total(ay, center, y0, m);
+  const long long plane = (long long)h * out_w;
+  const float* p = mid + (long long)y0 * out_w + ox;
+  float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+  for (int j = 0; j < m; ++j, p += out_w) {
+    const float wt = aa_weight(ay, center, y0 + j, total);
+    if (j == 0) {
+      a0 = __fmul_rn(p[0], wt); a1 = __fmul_rn(p[plane], wt); a2 = __fmul_rn(p[2 * plane], wt);
+    } else {
+      a0 = __fmaf_rn(p[0], wt, a0); a1 = __fmaf_rn(p[plane], wt, a1); a2 = __fmaf_rn(p[2 * plane], wt, a2);
+    }
+  }
+  dst[i] = a0;
+  dst[n + i] = a1;
+  dst[2 * n + i] = a2;
+}
+
+// Palette mask u8 [h, w] -> int64 [out_h, out_w] through host-built source rows / columns (negative = outside,
+// written as 0): Pillow's NEAREST resize is a pure gather once its index tables are known.
+__global__ void __launch_bounds__(256)
+resize_labels_kernel(const unsigned char* __restrict__ src, long long* __restrict__ dst, int w, int out_w,
+                     long long n, const int* __restrict__ src_y, const int* __restrict__ src_x) {
+  const long long i = blockIdx.x * 256ll + threadIdx.x;
+  if (i >= n) return;
+  const int oy = (int)(i / out_w), ox = (int)(i - (long long)oy * out_w);
+  const int y = src_y[oy], x = src_x[ox];
+  dst[i] = (y < 0 || x < 0) ? 0 : src[(long long)y * w + x];
 }
 }  // namespace ew
 
@@ -994,6 +1141,51 @@ int ew_prob_to_ids(const float* prob, int c, int h, int w, int out_h, int out_w,
   const long long n = (long long)out_h * out_w;
   ew::prob_to_ids_kernel<<<(unsigned)ceil_div(n, 256ll), 256, 0, s>>>(prob, c, h, w, out_h, out_w, flip, (float)h / out_h,
                                                                      (float)w / out_w, lut, out_u8, out_i64);
+  B200_LAUNCH_CHECK();
+  return 0;
+}
+size_t ew_resize_rgb8_workspace_bytes(int h, int out_w, int mode) {
+  return mode == RESIZE_READER ? sizeof(float) * 3 * (size_t)h * out_w : 0;
+}
+int ew_resize_rgb8(const unsigned char* src, float* dst, float* ws, int h, int w, int out_h, int out_w, int mode,
+                   const float* mean, const float* stdv, cudaStream_t s) {
+  B200_REQUIRE(src && dst && h > 0 && w > 0 && out_h > 0 && out_w > 0 && mean && stdv, "resize_rgb8: bad arguments");
+  B200_REQUIRE(mode == RESIZE_READER || mode == RESIZE_DEMO, "resize_rgb8: unknown mode %d", mode);
+  B200_REQUIRE(mode == RESIZE_DEMO || ws, "resize_rgb8: reader mode needs a workspace");
+  const long long n = (long long)out_h * out_w;
+  if (mode == RESIZE_DEMO) {
+    ew::resize_bilinear_rgb8_kernel<<<(unsigned)ceil_div(n, 256ll), 256, 0, s>>>(
+        src, dst, h, w, out_h, out_w, (float)h / out_h, (float)w / out_w, mean[0], mean[1], mean[2], stdv[0], stdv[1],
+        stdv[2]);
+    B200_LAUNCH_CHECK();
+    return 0;
+  }
+  ew::resize_aa_rows_rgb8_kernel<<<(unsigned)ceil_div((long long)h * out_w, 256ll), 256, 0, s>>>(
+      src, ws, h, w, out_w, ew::aa_axis(w, out_w), mean[0], mean[1], mean[2], stdv[0], stdv[1], stdv[2]);
+  B200_LAUNCH_CHECK();
+  ew::resize_aa_cols_kernel<<<(unsigned)ceil_div(n, 256ll), 256, 0, s>>>(ws, dst, h, out_h, out_w,
+                                                                          ew::aa_axis(h, out_h));
+  B200_LAUNCH_CHECK();
+  return 0;
+}
+int ew_resize_aa_weights(int n_in, int n_out, int max_taps, int* x0, int* n, float* wt) {
+  B200_REQUIRE(n_in > 0 && n_out > 0 && max_taps > 0 && x0 && n && wt, "resize_aa_weights: bad arguments");
+  const ew::AaAxis a = ew::aa_axis(n_in, n_out);
+  B200_REQUIRE(a.max_taps <= max_taps, "resize_aa_weights: %d -> %d needs max_taps >= %d", n_in, n_out, a.max_taps);
+  for (int i = 0; i < n_out; ++i) {
+    float center;
+    ew::aa_window(a, i, center, x0[i], n[i]);
+    const float total = ew::aa_total(a, center, x0[i], n[i]);
+    for (int j = 0; j < max_taps; ++j)
+      wt[(long long)i * max_taps + j] = j < n[i] ? ew::aa_weight(a, center, x0[i] + j, total) : 0.f;
+  }
+  return 0;
+}
+int ew_resize_labels(const unsigned char* src, long long* dst, int h, int w, int out_h, int out_w, const int* src_y,
+                     const int* src_x, cudaStream_t s) {
+  B200_REQUIRE(src && dst && src_y && src_x && h > 0 && w > 0 && out_h > 0 && out_w > 0, "resize_labels: bad arguments");
+  const long long n = (long long)out_h * out_w;
+  ew::resize_labels_kernel<<<(unsigned)ceil_div(n, 256ll), 256, 0, s>>>(src, dst, w, out_w, n, src_y, src_x);
   B200_LAUNCH_CHECK();
   return 0;
 }

@@ -30,4 +30,11 @@ int ew_transpose_append(const __half* src, __half* dst, long long ld_dst, int n,
 int ew_ingest_rgb8(const unsigned char* src, float* dst, int h, int w, const float* mean, const float* stdv, cudaStream_t s);
 int ew_prob_to_ids(const float* prob, int c, int h, int w, int out_h, int out_w, int flip, const int* lut,
                    unsigned char* out_u8, long long* out_i64, cudaStream_t s);
+enum { RESIZE_READER = 0, RESIZE_DEMO = 1 };  // == DEVA_B200_RESIZE_READER / _DEMO
+size_t ew_resize_rgb8_workspace_bytes(int h, int out_w, int mode);
+int ew_resize_rgb8(const unsigned char* src, float* dst, float* ws, int h, int w, int out_h, int out_w, int mode,
+                   const float* mean, const float* stdv, cudaStream_t s);
+int ew_resize_aa_weights(int n_in, int n_out, int max_taps, int* x0, int* n, float* wt);
+int ew_resize_labels(const unsigned char* src, long long* dst, int h, int w, int out_h, int out_w, const int* src_y,
+                     const int* src_x, cudaStream_t s);
 }  // namespace b200

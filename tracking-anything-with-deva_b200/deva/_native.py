@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), 'csrc', 'libdeva_b200.so')
-ABI_VERSION = 11
+ABI_VERSION = 12
 LIST_PITCH = 32
 MAX_GROUPS = 256
 
@@ -96,6 +96,11 @@ _SIGNATURES = {
                                       ctypes.POINTER(ctypes.c_float), c_void_p]),
     'deva_b200_prob_to_ids': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                       c_void_p]),
+    'deva_b200_resize_rgb8_workspace_bytes': (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+    'deva_b200_resize_rgb8': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+                                      ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float), c_void_p]),
+    'deva_b200_resize_aa_weights': (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    'deva_b200_resize_labels': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
 }
 EXPORTS = tuple(_SIGNATURES.keys())
 
@@ -359,6 +364,35 @@ def ingest_rgb8(src, dst, h, w, mean, std):
 def prob_to_ids(prob, c, h, w, out_h, out_w, flip, lut, out_u8, out_i64):
     _check(lib().deva_b200_prob_to_ids(_ptr(prob), c, h, w, out_h, out_w, int(flip), _p(lut), _p(out_u8), _p(out_i64),
                                        _stream()), 'prob_to_ids')
+
+
+RESIZE_MODES = {'reader': 0, 'demo': 1}  # DEVA_B200_RESIZE_READER / _DEMO
+
+
+def resize_rgb8_workspace_bytes(h, w, out_h, out_w, mode):
+    return lib().deva_b200_resize_rgb8_workspace_bytes(h, w, out_h, out_w, RESIZE_MODES[mode])
+
+
+def resize_rgb8(src, dst, ws, h, w, out_h, out_w, mode, mean, std):
+    m = (ctypes.c_float * 3)(*[float(v) for v in mean])
+    s = (ctypes.c_float * 3)(*[float(v) for v in std])
+    _check(lib().deva_b200_resize_rgb8(_ptr(src), _ptr(dst), _p(ws), h, w, out_h, out_w, RESIZE_MODES[mode], m, s,
+                                       _stream()), 'resize_rgb8')
+
+
+def resize_aa_weights(n_in, n_out):
+    """Host tap tables of the antialiased resize n_in -> n_out: (x0 int32 [n_out], n int32 [n_out], w fp32 [n_out, T])."""
+    taps = 2 * (n_in // n_out + 2) + 1  # >= 2 * ceil(max(n_in / n_out, 1)) + 1
+    x0 = torch.empty(n_out, dtype=torch.int32)
+    n = torch.empty(n_out, dtype=torch.int32)
+    w = torch.empty(n_out, taps, dtype=torch.float32)
+    _check(lib().deva_b200_resize_aa_weights(n_in, n_out, taps, _ptr(x0), _ptr(n), _ptr(w)), 'resize_aa_weights')
+    return x0, n, w
+
+
+def resize_labels(src, dst, h, w, out_h, out_w, src_y, src_x):
+    _check(lib().deva_b200_resize_labels(_ptr(src), _ptr(dst), h, w, out_h, out_w, _ptr(src_y), _ptr(src_x), _stream()),
+           'resize_labels')
 
 
 def transpose_append(src, dst, ld_dst, n, c):
